@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one rank per GPU under torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the CPU arm: the oracle port on the box's host cores
+    python bench.py ... --dump-outputs DIR                   # also write the film and counters of the timed steps (dump_outputs)
 
 Workload (BASELINE.json configs[3], SURVEY §8d C4): synthetic 1M-triangle random mesh inside the Cornell walls,
 1920x1080, one 4096-spp frame rendered in additive passes. One STEP = one pass of `--spp-per-step` samples per pixel
@@ -53,7 +54,26 @@ def parse():
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of the bounded cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned after its last step as DIR/<name>.npy")
     return ap.parse_args()
+
+
+DUMP_PIXELS = 1 << 21   # 32 MiB of RGBW float32 (+ 16 MiB of float64 indices when sampled): the default 1920x1080 film goes whole
+
+
+def dump_outputs(path, film, stats):
+    """film.npy: the RGBW film the timed passes accumulated from zero (H x W x 4 float32; above DUMP_PIXELS pixels a fixed, seeded
+    sample of them, N x 4, with their flat indices in film_pixel_index.npy); counters.npy: the trb_stats ray and test
+    counters of the timed steps (float64; the two timing fields of trb_stats are left out). The film is summed with float
+    atomics, so two runs agree to float32 rounding of those sums; the counters agree exactly."""
+    os.makedirs(path, exist_ok=True)
+    px = film.reshape(-1, 4)
+    if len(px) > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(len(px), DUMP_PIXELS, replace=False))
+        np.save(os.path.join(path, "film_pixel_index.npy"), idx.astype(np.float64))
+        film = px[idx]
+    np.save(os.path.join(path, "film.npy"), film.astype(np.float32))
+    np.save(os.path.join(path, "counters.npy"), stats[:8].astype(np.float64))
 
 
 def alg_bytes(rays, node, tri, inst):
@@ -258,7 +278,7 @@ def run_ours(a):
         step(i)
     if comm:
         comm.reduce_film(film.data_ptr(), film.numel(), 0, stream)     # warm the communicator
-        film.zero_()                                                    # the timed passes accumulate one frame's film from zero on every rank
+    film.zero_()                                                        # the timed passes accumulate one frame's film from zero on every rank
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
@@ -290,6 +310,8 @@ def run_ours(a):
     total_ms = max_over_ranks(e_begin.elapsed_time(e_end), dev)
     kernel_ms = [kev[k][0].elapsed_time(kev[k][1]) for k in range(a.steps)]
     st = stats.cpu().numpy()
+    if rank == 0 and a.dump_outputs:   # before the film buffer is reused below; rank 0 holds the reduced film
+        dump_outputs(a.dump_outputs, film.cpu().numpy(), st)
     tot = sum_over_ranks([st[0], st[1], st[2], st[3], st[4]], dev)     # samples, primary, shadow, mis, continuation (all ranks)
     rays_all = sum(tot[1:5])
 

@@ -3,14 +3,15 @@
 tr15.json references 13 OBJ files (cone, teapot, teapot2, u_logo, buddha, dragon, rust_logo, lucy, ajax, cow and three
 kenny_nl trees) and 5 MERL BRDF files that are NOT in the reference repository (SURVEY §8d). This script
 
-  * fixture():  re-serialises /root/reference/scenes/tr15.json (when present) into tests/golden/scenes/c5_tr15.json —
+  * fixture(scenes): re-serialises tr15.json from a tray_rust checkout's scenes/ directory into tests/golden/scenes/c5_tr15.json
+                (and logo_shadow / logo_with_friends / suzanne_scene.json, which only the loader test reads) —
                 the scene DESCRIPTION (camera / group / object keyframes, materials, lights) is the reference's, unchanged;
   * write_assets(root): generates, next to that JSON, procedural OBJ files carrying the model names tr15.json asks for
                 (closed noisy icospheres / cones with normals and uvs, sized like the originals' roles: ~80 k triangles for the
                 scanned statues, a few thousand for props) and MERL-format binaries from analytic lobes (one tint per file).
                 ~190 MB, generated where needed (GPU box, CPU tests), never committed.
 
-    python tests/golden/make_tr15.py            # refresh the fixture and write the assets
+    python tests/golden/make_tr15.py [--force] [SCENES]   # write the assets; with SCENES, refresh the fixtures from it first
 """
 import json
 import math
@@ -23,8 +24,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, REPO)
 SCENES = os.path.join(HERE, "scenes")
-FIXTURE = os.path.join(SCENES, "c5_tr15.json")
-REFERENCE = "/root/reference/scenes/tr15.json"
+FIXTURES = {"tr15.json": "c5_tr15.json", "logo_shadow.json": "logo_shadow.json", "logo_with_friends.json": "logo_with_friends.json",
+            "suzanne_scene.json": "suzanne_scene.json"}
 
 # file -> [(model name, kind, subdivisions, anisotropic scale, noise, seed)]
 MODELS = {
@@ -52,13 +53,11 @@ MERL = {"brdfs/black-oxidized-steel.binary": (0.25, 0.25, 0.27, 0.03), "brdfs/si
         "brdfs/brass.binary": (0.85, 0.65, 0.35, 0.04)}
 
 
-def fixture():
-    """Refresh tests/golden/scenes/c5_tr15.json from the reference (only possible where /root/reference exists)."""
-    if not os.path.exists(REFERENCE):
-        return False
-    d = json.load(open(REFERENCE))
-    json.dump(d, open(FIXTURE, "w"), separators=(",", ":"))
-    return True
+def fixture(scenes):
+    """Refresh the scene fixtures under tests/golden/scenes from `scenes`, the scenes/ directory of a tray_rust checkout."""
+    for src, dst in FIXTURES.items():
+        d = json.load(open(os.path.join(scenes, src)))
+        json.dump(d, open(os.path.join(SCENES, dst), "w"), separators=(",", ":"))
 
 
 def cone_mesh(segments):
@@ -135,5 +134,8 @@ def write_assets(root=SCENES, force=False):
 
 
 if __name__ == "__main__":
-    print("fixture refreshed from the reference:", fixture())
+    ref = [a for a in sys.argv[1:] if a != "--force"]
+    if ref:
+        fixture(ref[0])
+        print("fixtures refreshed from", ref[0])
     print("assets under", write_assets(force="--force" in sys.argv))

@@ -1,12 +1,12 @@
 """Independent check of the loader half of the drop-in (VERDICT r01 "parity is self-referential above the ABI"): every scene
 file the reference ships is flattened twice — by the product's C++ loader (trb_desc_load_json) and by tests/loader_ref.py
-(numpy restatement of /root/reference/src/scene.rs + keyframe.rs with LAPACK's SVD) — and compared field by field:
+(numpy restatement of tray_rust's src/scene.rs + keyframe.rs with LAPACK's SVD) — and compared field by field:
 instance order / kinds / shapes / parameters, transform stacks (group levels, B-spline degree and knots), every TRS keyframe
 of the f64-SVD polar decomposition, colour keys, materials, cameras, film, OBJ vertex unification and the MERL import.
 
-The scene JSONs are read from /root/reference/scenes when that tree exists (this container); on a box without it the three
-committed fixtures (c1, c2, c5_tr15 — re-serialised copies) are used. Assets that the reference repository does not contain
-(every OBJ but cube.obj, every MERL file) are generated stand-ins (tests/golden/make_tr15.py)."""
+The scene JSONs are the committed fixtures under tests/golden/scenes: re-serialised copies of the six files in tray_rust's
+scenes/ directory (tests/golden/make_tr15.py). Assets that the reference repository does not contain (every OBJ but
+cube.obj, every MERL file) are generated stand-ins (tests/golden/make_tr15.py)."""
 import ctypes as C
 import json
 import os
@@ -24,18 +24,14 @@ sys.path.insert(0, os.path.join(HERE, "golden"))
 import loader_ref as LR  # noqa: E402
 import make_tr15  # noqa: E402
 
-REF = "/root/reference/scenes"
-FIXTURES = {"cornell_box": "c1_cornell_box.json", "smallpt": "c2_smallpt.json", "tr15": "c5_tr15.json"}
-SCENES = ["cornell_box", "smallpt", "logo_shadow", "logo_with_friends", "suzanne_scene", "tr15"]
+FIXTURES = {"cornell_box": "c1_cornell_box.json", "smallpt": "c2_smallpt.json", "logo_shadow": "logo_shadow.json",
+            "logo_with_friends": "logo_with_friends.json", "suzanne_scene": "suzanne_scene.json", "tr15": "c5_tr15.json"}
+SCENES = list(FIXTURES)
 
 
 def stage(name, tmp):
     """Copy the scene JSON into tmp and put stand-in assets where its relative paths point."""
-    src = os.path.join(REF, name + ".json")
-    if not os.path.exists(src):
-        if name not in FIXTURES:
-            pytest.skip("needs /root/reference/scenes/%s.json" % name)
-        src = os.path.join(HERE, "golden", "scenes", FIXTURES[name])
+    src = os.path.join(HERE, "golden", "scenes", FIXTURES[name])
     dst = os.path.join(tmp, name + ".json")
     shutil.copy(src, dst)
     d = json.load(open(dst))
